@@ -142,6 +142,39 @@ def count_tokens(L, state):
     return n
 
 
+def collect_outputs(L, states):
+    """what a caller of the timed path receives for each chunk: its tokens with their probabilities and the segment times, as arrays
+    padded to the longest chunk (n_tokens / n_segments hold the true lengths)"""
+    L.whisper_full_get_token_data_from_state.restype = load_pkg().TokenData
+    L.whisper_full_get_token_data_from_state.argtypes = [C.c_void_p, C.c_int, C.c_int]
+    toks, segs = [], []
+    for st in states:
+        n_seg = L.whisper_full_n_segments_from_state(st)
+        segs.append([(L.whisper_full_get_segment_t0_from_state(st, s), L.whisper_full_get_segment_t1_from_state(st, s)) for s in range(n_seg)])
+        toks.append([L.whisper_full_get_token_data_from_state(st, s, j) for s in range(n_seg) for j in range(L.whisper_full_n_tokens_from_state(st, s))])
+    n_tok = max(1, max(len(t) for t in toks)); n_seg = max(1, max(len(s) for s in segs))
+    arrays = {"token_ids": np.full((len(toks), n_tok), -1.0), "token_p": np.zeros((len(toks), n_tok), np.float32),
+              "token_plog": np.zeros((len(toks), n_tok), np.float32), "n_tokens": np.array([len(t) for t in toks], np.float64),
+              "segment_t0": np.full((len(segs), n_seg), -1.0), "segment_t1": np.full((len(segs), n_seg), -1.0),
+              "n_segments": np.array([len(s) for s in segs], np.float64)}
+    for i, t in enumerate(toks):
+        arrays["token_ids"][i, :len(t)] = [d.id for d in t]
+        arrays["token_p"][i, :len(t)] = [d.p for d in t]
+        arrays["token_plog"][i, :len(t)] = [d.plog for d in t]
+    for i, s in enumerate(segs):
+        arrays["segment_t0"][i, :len(s)] = [a for a, _ in s]
+        arrays["segment_t1"][i, :len(s)] = [b for _, b in s]
+    return arrays
+
+
+def dump_outputs(arrays, out_dir, rank):
+    """<out_dir>/<name>.npy for each array of collect_outputs"""
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "_rank%d" % rank if rank else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+
+
 def ref_threads():
     """thread budget of the reference CPU arm: all logical CPUs (WB200_REF_THREADS overrides)"""
     if os.environ.get("WB200_REF_THREADS"):
@@ -258,7 +291,8 @@ def run_config2(args, local):
 
 
 def run_config3(args, local):
-    """BASELINE configs[2]: large-v3 Q4_K, single B200, beam_size 5, ONE 30-minute synthetic clip (60 x the 30 s generator, seeds 1234+i), whisper_full"""
+    """BASELINE configs[2]: large-v3 Q4_K, single B200, beam_size 5, ONE 30-minute synthetic clip (60 x the 30 s generator, seeds 1234+i), whisper_full;
+    a step is one whisper_full call on the whole clip"""
     import torch
     pkg = load_pkg(); synth = pkg.synth
     model = synth.cached_model("large-v3", synth.Q4_K, seed=0, fast_pool=True)
@@ -267,18 +301,23 @@ def run_config3(args, local):
     n_tiles = max(1, int(round(minutes * 2)))
     pcm = torch.from_numpy(np.concatenate([synth.synth_audio(seed=1234 + i, seconds=30.0) for i in range(n_tiles)])).pin_memory()
     p = L.whisper_full_default_params(1); p.print_progress = False; p.beam_search.beam_size = 5; p.temperature_inc = 0.0; p.n_threads = 4
-    c0 = (C.c_double * 8)(); L.wb200_counters(c0, 8)
-    L.whisper_reset_timings(eng.ctx)
-    torch.cuda.synchronize(); t0 = time.perf_counter()
-    assert L.whisper_full(eng.ctx, p, C.c_void_p(pcm.data_ptr()), pcm.numel()) == 0
-    torch.cuda.synchronize(); dt = time.perf_counter() - t0
+    times = []
+    for it in range(args.warmup + args.steps):
+        if it == args.warmup:
+            c0 = (C.c_double * 8)(); L.wb200_counters(c0, 8)
+        L.whisper_reset_timings(eng.ctx)
+        torch.cuda.synchronize(); t0 = time.perf_counter()
+        assert L.whisper_full(eng.ctx, p, C.c_void_p(pcm.data_ptr()), pcm.numel()) == 0
+        torch.cuda.synchronize(); times.append(time.perf_counter() - t0)
     c1 = (C.c_double * 8)(); L.wb200_counters(c1, 8)
+    cd = [(c1[i] - c0[i]) / args.steps for i in range(8)]          # per timed step
+    dt = float(np.mean(times[args.warmup:]))
     tm = _timings(L, eng.ctx)
     audio = pcm.numel() / 16000.0
-    out = {"metric": "xRT (audio-s/wall-s)", "value": audio / dt, "unit": "x real time", "n_gpus": 1, "steps": 1, "warmup": 0, "ms_per_step": 1e3 * dt,
+    out = {"metric": "xRT (audio-s/wall-s)", "value": audio / dt, "unit": "x real time", "n_gpus": 1, "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * dt,
            "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f16 tcgen05 (encode) / int8 block dot (decode), f32 accumulate", "data": "synthetic",
            "config": {"workload": "BASELINE configs[2]: large-v3 Q4_K (synthetic weights), beam_size 5, one %.0f-minute clip, whisper_full with host PCM (sequential windows: one stream)" % (audio / 60)},
-           "encode_ms": tm["encode_ms"], "batchd_ms_per_token": tm["batchd_ms"], "sample_ms": tm["sample_ms"], "windows": c1[5] - c0[5], "decode_passes": c1[0] - c0[0], "rows_per_pass": (c1[1] - c0[1]) / max(1.0, c1[0] - c0[0]),
+           "encode_ms": tm["encode_ms"], "batchd_ms_per_token": tm["batchd_ms"], "sample_ms": tm["sample_ms"], "windows": cd[5], "decode_passes": cd[0], "rows_per_pass": cd[1] / max(1.0, cd[0]),
            "decoded_tokens": sum(L.whisper_full_n_tokens(eng.ctx, i) for i in range(L.whisper_full_n_segments(eng.ctx))),
            "e2e": {"value": audio / dt, "unit": "x real time", "h2d_bytes_per_step": pcm.numel() * 4, "d2h_bytes_per_step": None}}
     print(json.dumps(out), flush=True)
@@ -348,7 +387,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ragged", action="store_true", help="skip the timestamps-on extra step")
     ap.add_argument("--config", type=int, default=4, choices=[2, 3, 4, 5], help="BASELINE.json configs[i-1]: 4 = the default line; 2, 3, 5 print their own JSON line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the tokens and segments of the last timed step as DIR/<name>.npy (default workload only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.config != 4):
+        ap.error("--dump-outputs applies to the default workload (--impl b200 --config 4)")
 
     rank = int(os.environ.get("RANK", "0")); local = int(os.environ.get("LOCAL_RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
@@ -399,9 +444,11 @@ def main():
     concat = torch.from_numpy(np.concatenate(pcms)).pin_memory()       # whisper_full_parallel input: one host buffer, sliced by the library
     states = []
 
-    def run_pass(mode):
+    def run_pass(mode, keep=False):
         """one step = all chunks of this rank.  mode "device": PCM resident in HBM (library queue driver); "parallel": one
-        whisper_full_parallel call on host PCM; "threads": one caller thread per chunk, whisper_full_with_state on its own state"""
+        whisper_full_parallel call on host PCM; "threads": one caller thread per chunk, whisper_full_with_state on its own state.
+        keep (device mode): copy the results into last["outputs"] before the states are freed, and the host time that takes into
+        last["keep_s"]"""
         if mode == "parallel":
             rc = L.whisper_full_parallel(eng.ctx, p, vp(concat.data_ptr()), concat.numel(), n_chunks)
             assert rc == 0, (rc, L.wb200_last_error())
@@ -425,10 +472,14 @@ def main():
         rc = L.wb200_full_batch_ex(eng.ctx, p, dev_ptrs, n_arr, n_chunks, outs, 1)
         assert rc == 0, (rc, L.wb200_last_error())
         last["tokens"] = sum(count_tokens(L, outs[i]) for i in range(n_chunks))
+        if keep:
+            t0 = time.perf_counter()
+            last["outputs"] = collect_outputs(L, [outs[i] for i in range(n_chunks)])
+            last["keep_s"] = time.perf_counter() - t0
         for i in range(n_chunks):
             L.whisper_free_state(outs[i])
 
-    def timed(mode, steps, warmup):
+    def timed(mode, steps, warmup, keep_last=False):
         for _ in range(warmup):
             run_pass(mode)
         if world > 1:
@@ -437,10 +488,10 @@ def main():
         h0, d0 = C.c_uint64(), C.c_uint64(); L.wb200_traffic(C.byref(h0), C.byref(d0))
         n0 = eng.launch_count()
         t0 = time.perf_counter()
-        for _ in range(steps):
-            run_pass(mode)
+        for i in range(steps):
+            run_pass(mode, keep=keep_last and i == steps - 1)
         torch.cuda.synchronize()
-        dt = time.perf_counter() - t0
+        dt = time.perf_counter() - t0 - last.pop("keep_s", 0.0)      # the copy for --dump-outputs is host work outside the step
         h1, d1 = C.c_uint64(), C.c_uint64(); L.wb200_traffic(C.byref(h1), C.byref(d1))
         launches = eng.launch_count() - n0
         dt = max_over_ranks(dt, world)
@@ -455,9 +506,11 @@ def main():
     for _ in range(args.warmup):
         run_pass("device")
     c0 = counters()
-    dt_res, launches, _, _ = timed("device", args.steps, 0)
+    dt_res, launches, _, _ = timed("device", args.steps, 0, keep_last=bool(args.dump_outputs))
     c1 = counters()
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(last.pop("outputs"), args.dump_outputs, rank)
     cd = [b - a for a, b in zip(c0, c1)]
     engine_stats = {"decode_passes_per_step": cd[0] / args.steps, "decode_rows_per_pass": cd[1] / max(cd[0], 1), "decode_gpu_ms_per_pass": cd[2] / max(cd[0], 1),
                     "decode_host_ms_per_pass": cd[3] / max(cd[0], 1), "encode_calls_per_step": cd[4] / args.steps, "encode_windows_per_step": cd[5] / args.steps,

@@ -9,7 +9,7 @@ import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 os.environ["WB200_DEBUG_TAPS"] = "1"
-from wbtest import load_lib, load_ref, DATA_DIR, read_wav_f32, F16, Q4_0, Q5_0, Q8_0, Q4_K, Q5_K, ref_quantize
+from wbtest import load_lib, load_ref, DATA_DIR, data_file, read_wav_f32, F16, Q4_0, Q5_0, Q8_0, Q4_K, Q5_K, ref_quantize
 from e2e_util import Side, synth, taps, rel_err, rms_err
 
 NAMES = {F16: "f16", Q4_0: "q4_0", Q5_0: "q5_0", Q8_0: "q8_0", Q4_K: "q4_k", Q5_K: "q5_k"}
@@ -20,7 +20,7 @@ def main():
     wtypes = [int(a) for a in sys.argv[2:]] or [F16, Q5_0]
     lib, ref = load_lib(), load_ref()
     lib.whisper_log_set(None, None) if False else None
-    stub = os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin" if cfg.endswith(".en") else "for-tests-ggml-tiny.bin")
+    stub = data_file("for-tests-ggml-tiny.en.bin" if cfg.endswith(".en") else "for-tests-ggml-tiny.bin")
     pcm = read_wav_f32(os.path.join(DATA_DIR, "jfk.wav"))
     tmp = tempfile.mkdtemp()
     for wt in wtypes:

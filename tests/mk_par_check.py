@@ -2,11 +2,11 @@
 import ctypes as C, os, sys, tempfile
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-from wbtest import DATA_DIR, Q5_0, load_lib
+from wbtest import data_file, Q5_0, load_lib
 from e2e_util import Side, synth
 
 path = os.path.join(tempfile.gettempdir(), "mk-par.bin")
-synth.write_model(path, "test-2l.en", Q5_0, seed=3, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+synth.write_model(path, "test-2l.en", Q5_0, seed=3, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
 pcm = synth.synth_audio(seed=9, seconds=60.0)
 A = Side(load_lib(), path, False); L = A.L
 fp = L.whisper_full_default_params(0); fp.print_progress = False; fp.temperature_inc = 0.0; fp.greedy.best_of = 1

@@ -2,12 +2,12 @@
 import os, sys, tempfile
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-from wbtest import DATA_DIR, Q5_0, load_lib
+from wbtest import data_file, Q5_0, load_lib
 from e2e_util import Side, synth
 
 wt = int(os.environ.get("WT", Q5_0))
 path = os.path.join(tempfile.gettempdir(), "mk-smoke-%d.bin" % wt)
-synth.write_model(path, "test-2l.en", wt, seed=7, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+synth.write_model(path, "test-2l.en", wt, seed=7, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
 A = Side(load_lib(), path, False)
 A.pcm_to_mel(synth.synth_audio(seed=1, seconds=2.0))
 A.encode(0)

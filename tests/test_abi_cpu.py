@@ -8,7 +8,7 @@ import subprocess
 
 import pytest
 
-from wbtest import ROOT, LIB_PATH, REF_PATH, DATA_DIR, bind_whisper_api, ContextParams, FullParams, TokenData, load_lib
+from wbtest import ROOT, LIB_PATH, REF_PATH, DATA_DIR, data_file, bind_whisper_api, ContextParams, FullParams, TokenData, load_lib
 
 
 def _exported(path):
@@ -84,11 +84,11 @@ def test_no_cpu_fallback_fails_loudly():
         pytest.skip("GPU present")
     L = bind_whisper_api(load_lib())
     cp = L.whisper_context_default_params()
-    ctx = L.whisper_init_from_file_with_params(os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin").encode(), cp)
+    ctx = L.whisper_init_from_file_with_params(data_file("for-tests-ggml-tiny.en.bin").encode(), cp)
     assert not ctx
     assert b"no CUDA device" in L.wb200_last_error() or b"CPU fallback" in L.wb200_last_error()
     cp.use_gpu = False
-    assert not L.whisper_init_from_file_with_params(os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin").encode(), cp)
+    assert not L.whisper_init_from_file_with_params(data_file("for-tests-ggml-tiny.en.bin").encode(), cp)
 
 
 C_PROGRAM = r"""
@@ -146,7 +146,7 @@ def test_unmodified_reference_cli_links_against_this_library(tmp_path):
     bound = re.findall(r"binding file \S*whisper-cli-b200 \[0\] to (\S+) \[0\]: normal symbol `(whisper_\w+)'", r.stderr + r.stdout)
     assert bound, "no whisper_* bindings seen"
     assert all(lib.endswith("libwhisper_b200.so") for lib, _ in bound), sorted({lib for lib, _ in bound})
-    model = os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"); wav = os.path.join(DATA_DIR, "jfk.wav")
+    model = data_file("for-tests-ggml-tiny.en.bin"); wav = os.path.join(DATA_DIR, "jfk.wav")
     r = subprocess.run([exe, "-m", model, "-f", wav], capture_output=True, text=True, timeout=120)
     import ctypes
     try:

@@ -12,7 +12,7 @@ import os
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, F16, TokenData, bind_whisper_api
+from wbtest import data_file, F16, TokenData, bind_whisper_api
 from e2e_util import synth
 
 vp = C.c_void_p
@@ -35,7 +35,7 @@ def test_predrawn_uniforms_consume_the_generators_like_the_reference_order(lib, 
     L = bind_whisper_api(lib)
     L.wb200_dbg_scripted_context.restype = vp; L.wb200_dbg_scripted_context.argtypes = [C.c_char_p]
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, (51864, 1500, 384, 6, 1, 448, 384, 6, 3, 80), F16, seed=5, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, (51864, 1500, 384, 6, 1, 448, 384, 6, 3, 80), F16, seed=5, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     pcm = (np.random.default_rng(3).standard_normal(int(seconds * 16000)) * 0.01).astype(np.float32)
     results = []
     for host_beam in (False, True):

@@ -4,7 +4,7 @@ libwhisper_b200.so (tests/test_zz_reference_cli_gpu.py) checks the engine, not t
 import os
 import pytest
 
-from wbtest import ROOT, DATA_DIR, F16
+from wbtest import ROOT, data_file, F16
 from e2e_util import synth
 from cli_util import check_cli_against_api, SILERO
 
@@ -18,7 +18,7 @@ def test_reference_cli_equals_reference_api(ref, tmp_path, vad):
     if vad and not os.path.exists(SILERO):
         pytest.skip("silero fixture missing")
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, "test-2l.en", F16, seed=7, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, "test-2l.en", F16, seed=7, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     got = check_cli_against_api(CLI_REF, ref, True, path, tmp_path, vad)
     assert sum(len(c["tokens"]) for c in got) > 50
 
@@ -30,7 +30,7 @@ def test_reference_bench_harness_on_reference(tmp_path):
     if not os.path.exists(exe):
         pytest.skip("oracle/_ref/whisper-bench-ref not built (make -C oracle cli)")
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, (51864, 1500, 384, 6, 1, 448, 384, 6, 1, 80), F16, seed=3, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, (51864, 1500, 384, 6, 1, 448, 384, 6, 1, 80), F16, seed=3, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     t = run_reference_bench(exe, path)
     print("reference whisper-bench on a 1-layer synthetic model:", {k: round(v[2], 2) for k, v in t.items()})
 
@@ -54,6 +54,6 @@ def test_reference_server_harness_on_reference(ref, tmp_path):
         pytest.skip("oracle/_ref/whisper-server-ref not built (make -C oracle cli)")
     pytest.importorskip("requests")
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, "test-2l.en", F16, seed=7, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, "test-2l.en", F16, seed=7, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     out = check_server_against_api(exe, ref, True, path)
     assert len(out["verbose_json"]["segments"]) >= 2                  # the 60-character wrap produced several segments

@@ -8,7 +8,7 @@ import os
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, F16, TokenData, bind_whisper_api, read_wav_f32
+from wbtest import DATA_DIR, data_file, F16, TokenData, bind_whisper_api, read_wav_f32
 from e2e_util import synth
 from test_full_scripted_cpu import Script, LOG_CB, _quiet
 
@@ -26,7 +26,7 @@ def test_dtw_host_math_matches_reference(lib, ref, tmp_path, preset):
     R = bind_whisper_api(ref)
     R.whisper_log_set.argtypes = [LOG_CB, vp]; R.whisper_log_set(_quiet, None)
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, (51864, 1500, 384, 6, 1, 448, 384, 6, 3, 80), F16, seed=9, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, (51864, 1500, 384, 6, 1, 448, 384, 6, 3, 80), F16, seed=9, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     cp = R.whisper_context_default_params(); cp.use_gpu = False; cp.flash_attn = False; cp.dtw_token_timestamps = True
     keep = None
     if preset == "custom":

@@ -17,7 +17,7 @@ import numpy as np
 import pytest
 
 os.environ["WB200_DEBUG_TAPS"] = "1"
-from wbtest import DATA_DIR, read_wav_f32, F16, Q4_0, Q5_0, Q8_0, Q4_K, Q5_K, ref_quantize
+from wbtest import DATA_DIR, data_file, read_wav_f32, F16, Q4_0, Q5_0, Q8_0, Q4_K, Q5_K, ref_quantize
 from e2e_util import Side, synth, taps, rms_err
 
 pytestmark = pytest.mark.gpu
@@ -159,7 +159,7 @@ def test_loader_fixtures_and_errors(lib):
     pcm = read_wav_f32(os.path.join(DATA_DIR, "jfk.wav"))
     for stub, nl in (("for-tests-ggml-tiny.en.bin", 4), ("for-tests-ggml-base.en.bin", 6), ("for-tests-ggml-tiny.bin", 4)):
         cp = L.whisper_context_default_params()
-        ctx = L.whisper_init_from_file_with_params(os.path.join(DATA_DIR, stub).encode(), cp)
+        ctx = L.whisper_init_from_file_with_params(data_file(stub).encode(), cp)
         assert ctx, L.wb200_last_error()
         assert L.whisper_model_n_audio_layer(ctx) == nl
         fp = L.whisper_full_default_params(0); fp.print_progress = False

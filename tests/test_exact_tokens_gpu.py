@@ -27,7 +27,7 @@ import os
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, F16, Q5_0, TokenData
+from wbtest import data_file, F16, Q5_0, TokenData
 from e2e_util import Side, synth
 
 pytestmark = pytest.mark.gpu
@@ -52,7 +52,7 @@ CASES = [(F16, 3, 1e-3, 100.0, 0, "exact"), (F16, 16, 1e-3, 100.0, 0, "exact"),
 
 
 def _model(tmp_path, wt, seed, attn, gain):
-    stub = os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin")
+    stub = data_file("for-tests-ggml-tiny.en.bin")
     path = str(tmp_path / ("cond-%d-%d-%g-%g.bin" % (wt, seed, attn, gain)))
     synth.write_model(path, "test-3l.en", wt, seed=seed, vocab_from=stub, scale=lambda n: synth.conditioned(n, attn, gain))
     return path

@@ -13,7 +13,7 @@ import zlib
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, F16, TokenData, bind_whisper_api
+from wbtest import DATA_DIR, data_file, F16, TokenData, bind_whisper_api
 from e2e_util import synth
 from test_grammar_cpu import build as build_grammar, lit, ALT, REF, CHAR, RNG
 from test_vad_cpu import SILERO
@@ -84,9 +84,14 @@ class Script:
         np.ctypeslib.as_array(logits, (V,))[:] = x
 
 
+def make_en_model(tmp_path):
+    en = str(tmp_path / "s1.en.bin")
+    synth.write_model(en, (51864, 1500, 384, 6, 1, 448, 384, 6, 1, 80), F16, seed=21, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
+    return en
+
+
 def make_models(tmp_path):
-    en = str(tmp_path / "s1.en.bin"); ml = str(tmp_path / "s1.multi.bin")
-    synth.write_model(en, (51864, 1500, 384, 6, 1, 448, 384, 6, 1, 80), F16, seed=21, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    en = make_en_model(tmp_path); ml = str(tmp_path / "s1.multi.bin")
     synth.write_model(ml, (51865, 1500, 384, 6, 1, 448, 384, 6, 1, 80), F16, seed=22, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.bin"))
     return en, ml
 

@@ -6,7 +6,7 @@ import os
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, FullParams, TokenData, bind_whisper_api
+from wbtest import data_file, FullParams, TokenData, bind_whisper_api
 
 vp = C.c_void_p
 END, ALT, REF, CHAR, NOT, RNG, CALT = range(7)
@@ -53,7 +53,7 @@ def test_grammar_filter_matches_reference(lib, ref, stub, gname):
     if not hasattr(ref, "wref_process_logits_grammar"):
         pytest.skip("oracle/_ref predates wref_process_logits_grammar (rebuild with make -C oracle)")
     L = bind_whisper_api(lib); R = bind_whisper_api(ref)
-    path = os.path.join(DATA_DIR, stub).encode()
+    path = data_file(stub).encode()
     cp = R.whisper_context_default_params(); cp.use_gpu = False
     rctx = R.whisper_init_from_file_with_params(path, cp)
     assert rctx

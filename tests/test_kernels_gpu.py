@@ -8,7 +8,7 @@ import os
 import numpy as np
 import pytest
 
-from wbtest import (F16, Q4_0, Q5_0, Q8_0, Q4_K, Q5_K, ref_quantize, bind_whisper_api, read_wav_f32, DATA_DIR,
+from wbtest import (F16, Q4_0, Q5_0, Q8_0, Q4_K, Q5_K, ref_quantize, bind_whisper_api, read_wav_f32, DATA_DIR, data_file,
                     parse_model_header)
 from oracle import ref_numpy as rn
 
@@ -28,7 +28,7 @@ def test_log_mel_matches_reference_on_jfk(lib, ref):
     ref.wref_mel_copy.argtypes = [vp, vp, C.c_int64]
     ref.wref_mel_n_len.argtypes = [vp]
     cp = ref.whisper_context_default_params(); cp.use_gpu = False
-    model = os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin")
+    model = data_file("for-tests-ggml-tiny.en.bin")
     ctx = ref.whisper_init_from_file_with_params(model.encode(), cp)
     _, filt = parse_model_header(model)
     pcm_full = read_wav_f32(os.path.join(DATA_DIR, "jfk.wav"))

@@ -9,7 +9,7 @@ import threading
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, Q5_0
+from wbtest import data_file, Q5_0
 from e2e_util import Side, synth
 
 pytestmark = pytest.mark.gpu
@@ -26,7 +26,7 @@ def _n_gpus():
 @pytest.mark.skipif(_n_gpus() < 2, reason="needs two GPUs (run under gpurun --gpus 2)")
 def test_states_spread_over_gpus_and_results_match_single_gpu(lib, tmp_path):
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, "test-2l.en", Q5_0, seed=5, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, "test-2l.en", Q5_0, seed=5, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     chunks = [synth.synth_audio(seed=70 + i, seconds=s) for i, s in enumerate((30.0, 12.0, 25.0, 7.0, 30.0, 18.0))]
 
     def run(multi):

@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 from wbtest import (F16, Q4_0, Q5_0, Q8_0, Q4_K, Q5_K, ref_quantize, ref_dequantize, bind_whisper_api, read_wav_f32,
-                    DATA_DIR, parse_model_header, ContextParams)
+                    DATA_DIR, data_file, parse_model_header, ContextParams)
 from oracle import ref_numpy as rn
 
 
@@ -53,7 +53,7 @@ def test_log_mel_float64_restatement_vs_reference(ref):
     assert n_len == (len(pcm) + 480000) // 160
     mel = np.empty((80, n_len), np.float32)
     assert ref.wref_mel_copy(st, mel.ctypes.data, mel.size) == 0
-    _, filt = parse_model_header(os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    _, filt = parse_model_header(data_file("for-tests-ggml-tiny.en.bin"))
     want = rn.log_mel(pcm, filt)
     assert want.shape == mel.shape
     # reference computes the FFT in f32: agreement to ~1e-4 except in bins far below the frame energy
@@ -90,7 +90,7 @@ def test_decoder_step_restatement_vs_reference(ref, tmp_path, wtype, tol):
     spec = importlib.util.spec_from_file_location("wb_synth", os.path.join(ROOT, "whisper.cpp_b200", "synth.py"))
     synth = importlib.util.module_from_spec(spec); spec.loader.exec_module(synth)
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, "test-2l.en", wtype, seed=7, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, "test-2l.en", wtype, seed=7, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     bind_whisper_api(ref)
     cp = ref.whisper_context_default_params(); cp.use_gpu = False
     ctx = ref.whisper_init_from_file_with_params(path.encode(), cp)
@@ -148,7 +148,7 @@ def test_encoder_restatement_vs_reference(ref, tmp_path, wtype, tol_enc, tol_kv)
     spec = importlib.util.spec_from_file_location("wb_synth", os.path.join(ROOT, "whisper.cpp_b200", "synth.py"))
     synth = importlib.util.module_from_spec(spec); spec.loader.exec_module(synth)
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, "test-2l.en", wtype, seed=7, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, "test-2l.en", wtype, seed=7, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     bind_whisper_api(ref)
     cp = ref.whisper_context_default_params(); cp.use_gpu = False
     ctx = ref.whisper_init_from_file_with_params(path.encode(), cp)

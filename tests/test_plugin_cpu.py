@@ -7,7 +7,7 @@ import os
 import subprocess
 import pytest
 
-from wbtest import ROOT, DATA_DIR, F16
+from wbtest import ROOT, DATA_DIR, data_file, F16
 from e2e_util import synth
 
 CLI = os.path.join(ROOT, "oracle", "_ref", "whisper-cli-ref")
@@ -27,7 +27,7 @@ def test_reference_cli_routes_all_four_graphs_to_the_plugin(tmp_path):
     if not (os.path.exists(CLI) and os.path.exists(PLUGIN)):
         pytest.skip("oracle/_ref/whisper-cli-ref or libggml-b200.so not built")
     model = str(tmp_path / "m.bin")
-    synth.write_model(model, "test-2l.en", F16, seed=7, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(model, "test-2l.en", F16, seed=7, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     env = dict(os.environ, GGML_BACKEND_PATH=PLUGIN, WB200_PLUGIN_DRY="1", WB200_PLUGIN_VERBOSE="1")
     r = subprocess.run([CLI, "-m", model, "-f", os.path.join(DATA_DIR, "jfk.wav"), "-bs", "1", "-bo", "1", "-nf", "-np", "-t", "2"],
                        capture_output=True, text=True, timeout=600, env=env)
@@ -46,7 +46,7 @@ def test_reference_bench_program_routes_its_graphs_to_the_plugin(tmp_path):
     if not (os.path.exists(exe) and os.path.exists(PLUGIN)):
         pytest.skip("oracle/_ref/whisper-bench-ref or libggml-b200.so not built")
     model = str(tmp_path / "m.bin")
-    synth.write_model(model, "test-2l.en", F16, seed=7, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(model, "test-2l.en", F16, seed=7, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     env = dict(os.environ, GGML_BACKEND_PATH=PLUGIN, WB200_PLUGIN_DRY="1", WB200_PLUGIN_VERBOSE="1")
     r = subprocess.run([exe, "-m", model, "-t", "2"], capture_output=True, text=True, timeout=600, env=env)
     assert r.returncode == 0, r.stderr[-1500:]

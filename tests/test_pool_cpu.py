@@ -16,7 +16,7 @@ import pytest
 
 from wbtest import F16, DATA_DIR
 from e2e_util import synth
-from test_full_scripted_cpu import Script, make_models, LOG_CB, _quiet
+from test_full_scripted_cpu import Script, make_en_model, LOG_CB, _quiet
 
 vp = C.c_void_p
 ENC_CB = C.CFUNCTYPE(C.c_bool, vp, vp, vp)
@@ -33,7 +33,7 @@ def test_concurrent_callers_on_the_scripted_pool(lib, tmp_path):
     L = bind_whisper_api(lib)
     L.whisper_log_set.argtypes = [LOG_CB, vp]; L.whisper_log_set(_quiet, None)
     L.wb200_dbg_scripted_context.restype = vp; L.wb200_dbg_scripted_context.argtypes = [C.c_char_p]
-    en, _ = make_models(tmp_path)
+    en = make_en_model(tmp_path)
     ctx = L.wb200_dbg_scripted_context(en.encode())
     assert ctx
     n = 10

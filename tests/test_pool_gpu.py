@@ -19,7 +19,7 @@ import threading
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, F16, Q5_0, FullParams, TokenData, read_wav_f32
+from wbtest import data_file, F16, Q5_0, FullParams, TokenData, read_wav_f32
 from e2e_util import Side, synth
 from test_full_scripted_cpu import Script, collect
 
@@ -28,7 +28,7 @@ vp = C.c_void_p
 
 
 def _model(tmp_path, cfg, wt, seed):
-    stub = os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin" if cfg.endswith(".en") else "for-tests-ggml-tiny.bin")
+    stub = data_file("for-tests-ggml-tiny.en.bin" if cfg.endswith(".en") else "for-tests-ggml-tiny.bin")
     path = str(tmp_path / f"{cfg}-{wt}-{seed}.bin")
     synth.write_model(path, cfg, wt, seed=seed, vocab_from=stub)
     return path

@@ -18,7 +18,7 @@ import os
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, F16, Q5_0
+from wbtest import data_file, F16, Q5_0
 from e2e_util import Side, synth, taps, rms_err
 
 vp = C.c_void_p
@@ -46,7 +46,7 @@ def _logits_and_taps(ref, path, nth, pcm, steps=6):
 @pytest.mark.parametrize("wt,enc_lo,log_lo", [(F16, 5e-5, 1e-2), (Q5_0, 1e-3, 1e-2)])
 def test_reference_differs_from_itself_across_thread_counts(ref, tmp_path, wt, enc_lo, log_lo):
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, "test-2l.en", wt, seed=7, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, "test-2l.en", wt, seed=7, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     pcm = synth.synth_audio(seed=512, seconds=30.0)
     t1, l1 = _logits_and_taps(ref, path, 1, pcm)
     t4, l4 = _logits_and_taps(ref, path, 4, pcm)

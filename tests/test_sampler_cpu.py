@@ -6,14 +6,14 @@ import os
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, FullParams, TokenData, bind_whisper_api
+from wbtest import data_file, FullParams, TokenData, bind_whisper_api
 
 vp = C.c_void_p
 
 
 def _setup(lib, ref, stub):
     L = bind_whisper_api(lib); R = bind_whisper_api(ref)
-    path = os.path.join(DATA_DIR, stub).encode()
+    path = data_file(stub).encode()
     cp = R.whisper_context_default_params(); cp.use_gpu = False
     rctx = R.whisper_init_from_file_with_params(path, cp)
     assert rctx

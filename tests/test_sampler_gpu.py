@@ -5,7 +5,7 @@ import os
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, FullParams, TokenData, bind_whisper_api
+from wbtest import data_file, FullParams, TokenData, bind_whisper_api
 
 pytestmark = pytest.mark.gpu
 vp = C.c_void_p
@@ -14,7 +14,7 @@ vp = C.c_void_p
 @pytest.mark.parametrize("stub", ["for-tests-ggml-tiny.en.bin", "for-tests-ggml-tiny.bin"])
 def test_device_sampler_matches_host_filter(lib, stub):
     L = bind_whisper_api(lib)
-    path = os.path.join(DATA_DIR, stub).encode()
+    path = data_file(stub).encode()
     sig = [C.POINTER(FullParams), C.POINTER(C.c_int), C.c_int, C.c_int, C.c_int]
     L.wb200_dbg_process_logits.argtypes = [C.c_char_p] + sig + [C.c_float, vp, vp, vp, vp, C.POINTER(TokenData)]
     L.wb200_dbg_greedy_sample.argtypes = [C.c_char_p] + sig + [vp, C.POINTER(TokenData)]
@@ -62,7 +62,7 @@ def test_device_categorical_draws_match_host_sampler(lib, stub):
     """beam search: the k draws of std::discrete_distribution(probs) per decoder (whisper_sample_token_topk, src/whisper.cpp:6545-6618) made
     on the device from host-drawn uniforms, against the host sampler (pinned to the reference bit for bit in test_sampler_cpu)."""
     L = bind_whisper_api(lib)
-    path = os.path.join(DATA_DIR, stub).encode()
+    path = data_file(stub).encode()
     sig = [C.POINTER(FullParams), C.POINTER(C.c_int), C.c_int, C.c_int, C.c_int]
     L.wb200_dbg_sample_topk.argtypes = [C.c_char_p] + sig + [C.c_float, vp, C.c_int, C.c_int, C.POINTER(TokenData)]
     L.wb200_dbg_draw_sample.argtypes = [C.c_char_p] + sig + [vp, C.c_int, C.c_int, C.POINTER(TokenData)]

@@ -7,7 +7,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from wbtest import ROOT, DATA_DIR, Q4_0, Q5_0, Q8_0, F16, ref_quantize, bind_whisper_api, parse_model_header
+from wbtest import ROOT, data_file, Q4_0, Q5_0, Q8_0, F16, ref_quantize, bind_whisper_api, parse_model_header
 
 spec = importlib.util.spec_from_file_location("wb_synth", os.path.join(ROOT, "whisper.cpp_b200", "synth.py"))
 synth = importlib.util.module_from_spec(spec); spec.loader.exec_module(synth)
@@ -24,7 +24,7 @@ def test_numpy_quantisers_bit_exact_vs_ggml(ref, wtype):
 
 @pytest.mark.parametrize("stub,n_mels", [("for-tests-ggml-tiny.en.bin", 80)])
 def test_mel_filterbank_matches_reference_model_files(stub, n_mels):
-    _, filt = parse_model_header(os.path.join(DATA_DIR, stub))
+    _, filt = parse_model_header(data_file(stub))
     mine = synth.mel_filters(n_mels)
     assert mine.shape == filt.shape
     assert np.abs(mine - filt).max() < 1e-6
@@ -34,7 +34,7 @@ def test_mel_filterbank_matches_reference_model_files(stub, n_mels):
 def test_written_model_loads_in_reference(ref, tmp_path, wtype):
     bind_whisper_api(ref)
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, "test-2l.en", wtype, seed=1, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, "test-2l.en", wtype, seed=1, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     cp = ref.whisper_context_default_params(); cp.use_gpu = False
     ctx = ref.whisper_init_from_file_with_params(path.encode(), cp)
     assert ctx
@@ -52,7 +52,7 @@ def test_host_expanded_formats_load_in_reference_and_parse_here(lib, ref, tmp_pa
     bind_whisper_api(ref); bind_whisper_api(lib)
     path = str(tmp_path / "m.bin")
     cfg = "test-2l-512.en" if wtype in (synth.Q2_K, synth.Q3_K, synth.Q6_K) else "test-2l.en"          # K-quants need rows of 256
-    synth.write_model(path, cfg, wtype, seed=1, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"), quantizer=lambda t, w: ref_quantize(ref, t, w))
+    synth.write_model(path, cfg, wtype, seed=1, vocab_from=data_file("for-tests-ggml-tiny.en.bin"), quantizer=lambda t, w: ref_quantize(ref, t, w))
     cp = ref.whisper_context_default_params(); cp.use_gpu = False
     ctx = ref.whisper_init_from_file_with_params(path.encode(), cp)
     assert ctx

@@ -6,7 +6,7 @@ import os
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, bind_whisper_api
+from wbtest import data_file, bind_whisper_api
 
 vp = C.c_void_p
 SIG = [vp, vp, vp, vp, C.c_int, C.c_int64, C.c_int64, vp, C.c_int, C.c_float, C.c_float, C.c_int, C.c_int, vp, vp, vp, vp, C.c_int]
@@ -29,7 +29,7 @@ def test_token_timestamps_and_wrapping_match_reference(lib, ref, stub):
     if not hasattr(ref, "wref_token_timestamps"):
         pytest.skip("oracle/_ref predates wref_token_timestamps (rebuild with make -C oracle)")
     R = bind_whisper_api(ref)
-    path = os.path.join(DATA_DIR, stub).encode()
+    path = data_file(stub).encode()
     cp = R.whisper_context_default_params(); cp.use_gpu = False
     rctx = R.whisper_init_from_file_with_params(path, cp)
     assert rctx

@@ -7,7 +7,7 @@ import os
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, Q5_0, bind_whisper_api, read_wav_f32
+from wbtest import DATA_DIR, data_file, Q5_0, bind_whisper_api, read_wav_f32
 from e2e_util import Side, synth
 from vad_synth import write_vad_model, speechy_audio
 from test_vad_cpu import bind_vad, ref_probs, GOLDEN, SILERO
@@ -81,7 +81,7 @@ def test_whisper_full_with_vad_cuts_the_same_audio(lib, ref, tmp_path):
     g = np.load(GOLDEN)
     vpath = SILERO.encode()
     mpath = str(tmp_path / "m.bin")
-    synth.write_model(mpath, "test-2l.en", Q5_0, seed=5, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(mpath, "test-2l.en", Q5_0, seed=5, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     pcm = np.ascontiguousarray(read_wav_f32(os.path.join(DATA_DIR, "jfk.wav")), np.float32)
     A, B = Side(lib, mpath, False), Side(ref, mpath, True)
     try:

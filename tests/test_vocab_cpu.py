@@ -4,7 +4,7 @@ import ctypes as C
 import os
 import pytest
 
-from wbtest import DATA_DIR, bind_whisper_api
+from wbtest import data_file, bind_whisper_api
 
 vp = C.c_void_p
 TEXTS = ["", " ", "hello world", " Hello, World!", "And so my fellow Americans, ask not what your country can do for you.",
@@ -14,7 +14,7 @@ TEXTS = ["", " ", "hello world", " Hello, World!", "And so my fellow Americans, 
 @pytest.mark.parametrize("stub", ["for-tests-ggml-tiny.en.bin", "for-tests-ggml-tiny.bin", "for-tests-ggml-large.bin"])
 def test_vocabulary_and_tokenizer_match_reference(lib, ref, stub):
     L = bind_whisper_api(lib); R = bind_whisper_api(ref)
-    path = os.path.join(DATA_DIR, stub).encode()
+    path = data_file(stub).encode()
     cp = R.whisper_context_default_params(); cp.use_gpu = False
     rctx = R.whisper_init_from_file_with_params(path, cp)
     assert rctx
@@ -58,7 +58,7 @@ def test_header_parser_rejects_bad_files(lib, tmp_path):
     """loader error paths that need no device (src/whisper.cpp:1497-1500, 1589-1600): bad magic, truncated header / vocabulary"""
     L = bind_whisper_api(lib)
     L.wb200_dbg_vocab_context.restype = vp; L.wb200_dbg_vocab_context.argtypes = [C.c_char_p]
-    good = open(os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"), "rb").read()
+    good = open(data_file("for-tests-ggml-tiny.en.bin"), "rb").read()
     cases = {"magic.bin": b"\x00\x01\x02\x03" + good[4:], "short_header.bin": good[:30], "short_vocab.bin": good[:4 + 44 + 8 + 80 * 201 * 4 + 4 + 1000],
              "empty.bin": b""}
     for name, blob in cases.items():

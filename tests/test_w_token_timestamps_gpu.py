@@ -9,7 +9,7 @@ import os
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, read_wav_f32, Q5_0, TokenData
+from wbtest import DATA_DIR, data_file, read_wav_f32, Q5_0, TokenData
 from e2e_util import Side, synth
 from test_full_scripted_cpu import Script
 
@@ -23,7 +23,7 @@ def test_token_timestamps_and_max_len(lib, ref, tmp_path, scripted):
     scripted = True: 3-text-layer model with the transcript scripted through logits_filter_callback (timestamps, several segments, host sampler)"""
     path = str(tmp_path / "m.bin")
     cfg = (51864, 1500, 384, 6, 1, 448, 384, 6, 3, 80) if scripted else "test-2l.en"
-    synth.write_model(path, cfg, Q5_0, seed=11, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, cfg, Q5_0, seed=11, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     pcm = read_wav_f32(os.path.join(DATA_DIR, "jfk.wav"))
     A = Side(lib, path, False)
     try:

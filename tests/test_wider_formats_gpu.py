@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 os.environ["WB200_DEBUG_TAPS"] = "1"
-from wbtest import DATA_DIR, read_wav_f32, ref_quantize
+from wbtest import DATA_DIR, data_file, read_wav_f32, ref_quantize
 from e2e_util import Side, synth, taps, rms_err
 
 pytestmark = pytest.mark.gpu
@@ -24,7 +24,7 @@ CASES = {synth.Q5_1: ("test-2l.en",     3e-2, 3.5e-2, 5e-2, 0.3), synth.Q4_1: ("
 def test_host_expanded_formats_match_reference(lib, ref, tmp_path, wt):
     cfg, e_enc, e_kv, e_log, margin = CASES[wt]
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, cfg, wt, seed=7, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"), quantizer=lambda t, w: ref_quantize(ref, t, w))
+    synth.write_model(path, cfg, wt, seed=7, vocab_from=data_file("for-tests-ggml-tiny.en.bin"), quantizer=lambda t, w: ref_quantize(ref, t, w))
     pcm = read_wav_f32(os.path.join(DATA_DIR, "jfk.wav"))
     A = Side(lib, path, False); B = Side(ref, path, True)
     try:
@@ -57,7 +57,7 @@ def test_kquants_expanded_to_f16_opt_in(lib, ref, tmp_path, monkeypatch, wt):
     monkeypatch.setenv("WB200_KQUANT_AS_F16", "1")
     e_enc, e_kv, e_log, margin = (4e-2, 5e-2, 7e-2, 0.4) if wt == synth.Q4_K else (3e-2, 3.5e-2, 5e-2, 0.3)     # tests/test_e2e_gpu.py TOL
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, "test-2l-512.en", wt, seed=7, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"), quantizer=lambda t, w: ref_quantize(ref, t, w))
+    synth.write_model(path, "test-2l-512.en", wt, seed=7, vocab_from=data_file("for-tests-ggml-tiny.en.bin"), quantizer=lambda t, w: ref_quantize(ref, t, w))
     pcm = read_wav_f32(os.path.join(DATA_DIR, "jfk.wav"))
     A = Side(lib, path, False); B = Side(ref, path, True)
     try:

@@ -13,13 +13,13 @@ import re
 import subprocess
 import pytest
 
-from wbtest import ROOT, DATA_DIR, F16, Q5_0
+from wbtest import ROOT, DATA_DIR, data_file, F16, Q5_0
 from e2e_util import synth
 
 pytestmark = pytest.mark.gpu
 CLI = os.path.join(ROOT, "oracle", "_ref", "whisper-cli-ref")
 PLUGIN = os.path.join(ROOT, "whisper.cpp_b200", "libggml-b200.so")
-STUB = os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin")
+STUB = data_file("for-tests-ggml-tiny.en.bin")
 
 
 CLI_DIRECT = os.path.join(ROOT, "oracle", "_ref", "whisper-cli-b200")     # the same CLI sources linked against libwhisper_b200.so (whisper.h boundary)

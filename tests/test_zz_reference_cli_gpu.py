@@ -6,7 +6,7 @@ The harness itself is validated on the CPU with the reference pair (tests/test_c
 import os
 import pytest
 
-from wbtest import ROOT, DATA_DIR, F16, Q5_0
+from wbtest import ROOT, data_file, F16, Q5_0
 from e2e_util import synth
 from cli_util import check_cli_against_api, SILERO
 
@@ -21,7 +21,7 @@ def test_reference_cli_runs_on_this_engine(lib, tmp_path, wt, vad):
     if vad and not os.path.exists(SILERO):
         pytest.skip("silero fixture missing")
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, "test-2l.en", wt, seed=7, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, "test-2l.en", wt, seed=7, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     check_cli_against_api(CLI, lib, False, path, tmp_path, vad)
 
 
@@ -33,7 +33,7 @@ def test_reference_bench_program_runs_on_this_engine(lib, tmp_path):
     if not os.path.exists(exe):
         pytest.skip("oracle/_ref/whisper-bench-b200 not built")
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, "test-2l.en", Q5_0, seed=7, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, "test-2l.en", Q5_0, seed=7, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     t = run_reference_bench(exe, path)
     print("whisper-bench on the engine (test-2l.en Q5_0):", {k: round(v[2], 3) for k, v in t.items()})
 
@@ -58,5 +58,5 @@ def test_reference_server_runs_on_this_engine(lib, tmp_path):
         pytest.skip("oracle/_ref/whisper-server-b200 not built")
     pytest.importorskip("requests")
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, "test-2l.en", Q5_0, seed=7, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, "test-2l.en", Q5_0, seed=7, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     check_server_against_api(exe, lib, False, path)

@@ -8,7 +8,7 @@ import os
 import numpy as np
 import pytest
 
-from wbtest import DATA_DIR, F16, Q5_0, TokenData, bind_whisper_api, read_wav_f32
+from wbtest import DATA_DIR, data_file, F16, Q5_0, TokenData, bind_whisper_api, read_wav_f32
 from e2e_util import synth
 from test_full_scripted_cpu import Script, LOG_CB, _quiet
 
@@ -38,7 +38,7 @@ def test_dtw_weights_and_timestamps(lib, ref, tmp_path, wt, tol):
     L = bind_whisper_api(lib); R = bind_whisper_api(ref)
     L.wb200_last_error.restype = C.c_char_p
     path = str(tmp_path / "m.bin")
-    synth.write_model(path, (51864, 1500, 384, 6, 1, 448, 384, 6, 3, 80), wt, seed=9, vocab_from=os.path.join(DATA_DIR, "for-tests-ggml-tiny.en.bin"))
+    synth.write_model(path, (51864, 1500, 384, 6, 1, 448, 384, 6, 3, 80), wt, seed=9, vocab_from=data_file("for-tests-ggml-tiny.en.bin"))
     pcm = np.ascontiguousarray(read_wav_f32(os.path.join(DATA_DIR, "jfk.wav")), np.float32)
     lctx, mine = _run(L, path, pcm, True)
     rctx, theirs = _run(R, path, pcm, False)

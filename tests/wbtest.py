@@ -83,6 +83,32 @@ def read_wav_f32(path):
 
 
 DATA_DIR = os.path.join(ROOT, "oracle", "_ref", "data")
+GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
+
+
+def data_file(name):
+    """path of a fixture of the reference's own tests: the copy kept in the repository (tests/golden/<name>.xz, unpacked into the
+    temp directory; a file already there is reused only if its bytes are the unpacked ones) when there is one, otherwise
+    oracle/_ref/data/<name> as build() copied it"""
+    packed = os.path.join(GOLDEN_DIR, name + ".xz")
+    if not os.path.exists(packed):
+        return os.path.join(DATA_DIR, name)
+    import lzma
+    import tempfile
+    with open(packed, "rb") as f:
+        data = lzma.decompress(f.read())
+    out_dir = os.path.join(tempfile.gettempdir(), "wb200-fixtures-%d" % os.getuid())
+    out = os.path.join(out_dir, name)
+    if os.path.exists(out):
+        with open(out, "rb") as f:
+            if f.read() == data:
+                return out
+    os.makedirs(out_dir, exist_ok=True)
+    tmp = "%s.tmp.%d" % (out, os.getpid())
+    with open(tmp, "wb") as g:
+        g.write(data)
+    os.replace(tmp, out)
+    return out
 
 
 def parse_model_header(path):
